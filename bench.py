@@ -4,6 +4,8 @@ frequency-bins x cadences / s; config[1] at N=1: 1024 Kepler long-cadence light 
 cadences, shared time grid) x 1e5 frequencies).
 
   python bench.py --gpus N --steps K --warmup W            # our arm (CUDA kernels via the C ABI)
+  python bench.py ... --dump-outputs DIR                   # also write the last step's power rows (rank 0, a
+                                                           #   fixed row sample) to DIR/power.npy
   python bench.py --impl reference ...                     # the reference's CPU algorithm (oracle port
                                                            #   of astropy LombScargle method="fast")
 For N > 1 launch with torchrun (one rank per GPU): the batch is sharded BY TARGET, every rank
@@ -442,6 +444,22 @@ def _peaks():
         return {}
 
 
+def power_sample(power, max_bytes=48 << 20, seed=0):
+    """Host copy of a fixed, seeded sample of the rows of a [B, F] float32 power tensor: every row when they fit in
+    `max_bytes`, else as many distinct rows (in ascending order) as do.  Same B, F and seed: same rows."""
+    import torch
+    B, F = power.shape
+    n = min(B, max(1, max_bytes // (4 * F)))
+    rows = np.arange(B) if n == B else np.sort(np.random.default_rng(seed).choice(B, n, replace=False))
+    return power.index_select(0, torch.as_tensor(rows, device=power.device)).cpu().numpy()
+
+
+def dump_outputs(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def _cores():
     try:
         return len(os.sched_getaffinity(0))
@@ -456,11 +474,12 @@ def _max_over_ranks(torch, dist, world, dev, vals):
     return [float(x) for x in tm.tolist()]
 
 
-def c5_step_stats(engine, torch, dist, rank, world, dev, times, fluxes, freq, steps, warmup, chunks=4):
+def c5_step_stats(engine, torch, dist, rank, world, dev, times, fluxes, freq, steps, warmup, chunks=4,
+                  sample_power=False):
     """Device-resident sharded ragged Lomb-Scargle (lightkurve_b200.dist.ShardedLombScargle): per step compute of this
     rank's shard + the pipelined all-gathers + restoring the target order.  Returns ms (device events, max over
     ranks) for the resident step and for the end-to-end step (pinned H2D of the shard, the step, D2H of the whole
-    gathered power array on every rank)."""
+    gathered power array on every rank); with `sample_power`, also `power_sample` of the last resident step's output."""
     from lightkurve_b200.dist import ShardedLombScargle
     job = ShardedLombScargle(times, fluxes, freq, "amplitude", chunks=chunks, device=dev)
     job.upload()
@@ -486,21 +505,27 @@ def c5_step_stats(engine, torch, dist, rank, world, dev, times, fluxes, freq, st
         out = job.run()
         h_out.copy_(out, non_blocking=True)
 
+    last = {}
+
+    def step_resident():
+        last["power"] = job.run()
+
     for _ in range(warmup):
         job.run()
     engine.profile_enable(True)
     l0 = engine.launch_count()
-    ms_res = timed(job.run, steps)
+    ms_res = timed(step_resident, steps)
     launches = (engine.launch_count() - l0) // max(1, steps)
     kms = engine.profile_read()
     engine.profile_enable(False)
+    sample = power_sample(last["power"]) if sample_power else None
     step_e2e()
-    ms_e2e = timed(step_e2e, max(2, steps // 2))
+    ms_e2e = timed(step_e2e, steps)
     k_ms = float(np.sum(kms)) / max(1, steps) if len(kms) else float("nan")      # all pieces of one step
     ms_res, ms_e2e, k_ms = _max_over_ranks(torch, dist, world, dev, [ms_res, ms_e2e, k_ms])
     mine = job.shards[rank]
     return dict(ms=ms_res, ms_e2e=ms_e2e, kernel_ms=k_ms, launches=int(launches), family=engine.ls_last_algo(),
-                h2d=job.h2d_bytes, d2h=int(job.n_total) * job.F * 4, n_local=len(mine), job=job)
+                h2d=job.h2d_bytes, d2h=int(job.n_total) * job.F * 4, n_local=len(mine), job=job, power_sample=sample)
 
 
 def _ragged_cpu_leg(times, fluxes, freq, n_lc=48, budget_s=12.0):
@@ -707,7 +732,7 @@ def run_c5(args, engine, torch, dist, rank, world, local_rank, dev):
     if sampler:
         sampler.start()
     st = c5_step_stats(engine, torch, dist, rank, world, dev, times, fluxes, freq, args.steps, args.warmup,
-                       chunks=args.chunks if args.chunks > 0 else 4)
+                       chunks=args.chunks if args.chunks > 0 else 4, sample_power=bool(args.dump_outputs) and rank == 0)
     clocks = sampler.stop() if sampler else None
     units = float(F) * float(sum(len(t) for t in times))
     if rank != 0:
@@ -733,6 +758,8 @@ def run_c5(args, engine, torch, dist, rank, world, local_rank, dev):
             "gpu_launches": st["launches"],
             "roofline": _ragged_roofline(F, units_local, st["kernel_ms"], st["family"], st["n_local"]),
             "cpu_baseline": cpu, "clocks": clocks}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"power": st["power_sample"]})
     print(json.dumps(line), flush=True)
 
 def nufft_leg_child(args):
@@ -823,7 +850,14 @@ def main():
     ap.add_argument("--nufft-leg", action="store_true", help=argparse.SUPPRESS)      # internal: child of secondary.ls_nufft
     ap.add_argument("--nufft-variants", action="store_true",
                     help="also time the NUFFT path's transform variants in a child process (secondary.ls_nufft)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the power rows of the last step (a fixed, seeded sample of at "
+                         "most 48 MB) to DIR/power.npy, float32, so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the CUDA path computed: it needs --impl ours")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -952,6 +986,8 @@ def main():
     clocks = sampler.stop() if sampler else None
     family = engine.ls_last_algo()             # what `auto` resolved to: "nufft", "tcgen05" or "simt"
     escalated = engine.ls_last_escalated()     # light curves of the last step that took the double-precision pass
+    # the last resident step's power rows (the path of the reported value), copied before the end-to-end steps run
+    dumped = power_sample(d_P) if args.dump_outputs and rank == 0 else None
 
     for _ in range(2):
         step_e2e()
@@ -1063,6 +1099,8 @@ def main():
             "gpu_launches": int(launches), "roofline": roofline, "cpu_baseline": cpu, "clocks": clocks,
             "secondary": secondary,
         }
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"power": dumped})
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
