@@ -151,6 +151,28 @@ int lkb_bls_power(const double* t, const double* y, const double* dy, const int6
                   double* transit_time, double* depth_snr, double* log_likelihood,
                   int32_t* best_bins, int mem, void* stream);
 
+/* K3s: the exact, unbinned search BoxLeastSquares(t, y, dy).power(period, duration,
+ * objective, method="slow", oversample) - lightkurve passes `method=` of
+ * to_periodogram("bls", ...) through to that call (periodogram.py:1169).  For each
+ * duration d, the transit epochs are t0_i = i*d/oversample (i < ceil((P + d/oversample)
+ * / (d/oversample))), a cadence is in the box when |((x - t0 + P/2) % P) - P/2| < d/2
+ * (x = t - min(t), numpy float semantics), and the FIRST strict maximum of the
+ * objective in (duration, t0) order with depth > 0 is kept.  duration_out is the
+ * trial duration itself.  Same arguments and layouts as lkb_bls_power, except:
+ *   times must be ascending within each light curve (else LKB_E_UNSUPPORTED);
+ *   best_index (nullable) int32 [B,P,3] = (duration index, t0 index, number of
+ *   in-box cadences) of the winning box.
+ * A period where no box has depth > 0 gets power = -inf, depth = depth_err =
+ * depth_snr = log_likelihood = duration = 0, transit_time = min(t), best_index =
+ * (-1, -1, 0); astropy raises there instead.
+ */
+int lkb_bls_power_slow(const double* t, const double* y, const double* dy, const int64_t* offsets, int B,
+                       const double* period, int64_t P, const double* duration, int D,
+                       int oversample, int objective,
+                       double* power, double* depth, double* depth_err, double* duration_out,
+                       double* transit_time, double* depth_snr, double* log_likelihood,
+                       int32_t* best_index, int mem, void* stream);
+
 /* Debug/parity entry: the per-sample bin index of bls.c for ONE period,
  * ind[n] = (int)(fabs(fmod(t[n]-min_t, period))/bin_duration)+1, evaluated by the
  * same device function the search kernel uses. */

@@ -46,6 +46,8 @@ SIGNATURES = {
                                     c_vp, c_int]),
     "lkb_bls_power": (c_int, [c_vp, c_vp, c_vp, c_vp, c_int, c_vp, c_i64, c_vp, c_int, c_int, c_int,
                               c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_vp]),
+    "lkb_bls_power_slow": (c_int, [c_vp, c_vp, c_vp, c_vp, c_int, c_vp, c_i64, c_vp, c_int, c_int, c_int,
+                                   c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_vp]),
     "lkb_bls_bin_index": (c_int, [c_vp, c_i64, c_dbl, c_dbl, c_dbl, c_vp, c_int, c_vp]),
     "lkb_flatten": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_dbl, c_int, c_dbl,
                             c_vp, c_vp, c_vp, c_int, c_vp]),

@@ -74,11 +74,11 @@ class LightCurveCollection(Collection):
                 return [lc.to_periodogram(method, **dict(kwargs)) for lc in self.data]
             res = engine.bls_power([p["time"] for p in preps], [p["flux"] for p in preps],
                                    None if p0["dy"] is None else [p["dy"] for p in preps], p0["period"],
-                                   p0["duration"], oversample=p0["oversample"], objective=p0["objective"])
+                                   p0["duration"], **BoxLeastSquaresPeriodogram._engine_kwargs(p0))
             out = []
             for b, p in enumerate(preps):
                 pg = BoxLeastSquaresPeriodogram._finish(p, res, b)
-                pg._dy = p["dy"]
+                pg._dy = p["lc_dy"]
                 out.append(pg)
             return out
         preps = [LombScarglePeriodogram._prepare(lc, **dict(kwargs)) for lc in self.data]

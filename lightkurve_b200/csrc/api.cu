@@ -216,6 +216,9 @@ int bls_power(const double*, const double*, const double*, const int64_t*, int, 
               const double*, int, int, int, double*, double*, double*, double*, double*, double*, double*, int32_t*,
               int, cudaStream_t);
 int bls_bin_index(const double*, int64_t, double, double, double, int32_t*, int, cudaStream_t);
+int bls_power_slow(const double*, const double*, const double*, const int64_t*, int, const double*, int64_t,
+                   const double*, int, int, int, double*, double*, double*, double*, double*, double*, double*,
+                   int32_t*, int, cudaStream_t);
 int flatten(const double*, const double*, const double*, const uint8_t*, const int64_t*, int, int, int, double, int,
             double, double*, double*, double*, int, cudaStream_t);
 int regress(const double*, int, const double*, const double*, const uint8_t*, const double*, const double*, int,
@@ -231,7 +234,7 @@ using namespace lkb;
 extern "C" {
 
 const char* lkb_last_error(void) { return t_err; }
-int lkb_version(void) { return 1000 * 0 + 1; }
+int lkb_version(void) { return 1000 * 0 + 2; }
 
 int lkb_device_count(void) {
   int n = 0;
@@ -351,6 +354,15 @@ int lkb_bls_power(const double* t, const double* y, const double* dy, const int6
   std::lock_guard<std::mutex> lk(g_mu);
   return bls_power(t, y, dy, offsets, B, period, P, duration, D, oversample, objective, power, depth, depth_err,
                    duration_out, transit_time, depth_snr, log_likelihood, best_bins, mem, (cudaStream_t)stream);
+}
+
+int lkb_bls_power_slow(const double* t, const double* y, const double* dy, const int64_t* offsets, int B,
+                       const double* period, int64_t P, const double* duration, int D, int oversample, int objective,
+                       double* power, double* depth, double* depth_err, double* duration_out, double* transit_time,
+                       double* depth_snr, double* log_likelihood, int32_t* best_index, int mem, void* stream) {
+  std::lock_guard<std::mutex> lk(g_mu);
+  return bls_power_slow(t, y, dy, offsets, B, period, P, duration, D, oversample, objective, power, depth, depth_err,
+                        duration_out, transit_time, depth_snr, log_likelihood, best_index, mem, (cudaStream_t)stream);
 }
 
 int lkb_bls_bin_index(const double* t_rel, int64_t N, double min_t, double period, double bin_duration,

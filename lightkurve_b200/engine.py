@@ -291,9 +291,14 @@ BLS_FIELDS = ("power", "depth", "depth_err", "duration", "transit_time", "depth_
 
 
 def bls_power(times, fluxes, flux_errs, period, duration, oversample=10, objective="likelihood",
-              return_bins=False):
-    """K3.  Lists of per-LC arrays (flux_errs: list or None => unit weights), one shared
-    period grid [P] and duration grid [D].  Returns dict of [B, P] float64 arrays."""
+              return_bins=False, method="fast"):
+    """K3 (method="fast", astropy's binned search) or K3s (method="slow", astropy's exact unbinned search; the times
+    of every light curve must be ascending).  Lists of per-LC arrays (flux_errs: list or None => unit weights), one
+    shared period grid [P] and duration grid [D].  Returns dict of [B, P] float64 arrays; with `return_bins`, also
+    "bins" [B, P, 2] = (start bin, duration in bins) for "fast" or "index" [B, P, 3] = (duration index, t0 index,
+    number of in-box cadences) for "slow"."""
+    if method not in ("fast", "slow"):
+        raise ValueError("method must be 'fast' or 'slow' (got %r)" % (method,))
     lib = L.load()
     B = len(times)
     t, offsets = _csr(times)
@@ -309,14 +314,24 @@ def bls_power(times, fluxes, flux_errs, period, duration, oversample=10, objecti
     duration = np.ascontiguousarray(np.atleast_1d(duration), dtype=np.float64)
     P, D = len(period), len(duration)
     outs = [np.empty((B, P), dtype=np.float64) for _ in range(7)]
-    bins = np.empty((B, P, 2), dtype=np.int32) if return_bins else None
-    L.check(lib.lkb_bls_power(L.ptr(t), L.ptr(y), L.ptr(dy), L.ptr(offsets), B, L.ptr(period), P, L.ptr(duration), D,
-                              int(oversample), L.BLS_SNR if objective == "snr" else L.BLS_LIKELIHOOD,
-                              *[L.ptr(o) for o in outs], L.ptr(bins), L.MEM_HOST, None))
+    if method == "slow":
+        index = np.empty((B, P, 3), dtype=np.int32) if return_bins else None
+        L.check(lib.lkb_bls_power_slow(L.ptr(t), L.ptr(y), L.ptr(dy), L.ptr(offsets), B, L.ptr(period), P,
+                                       L.ptr(duration), D, int(oversample),
+                                       L.BLS_SNR if objective == "snr" else L.BLS_LIKELIHOOD,
+                                       *[L.ptr(o) for o in outs], L.ptr(index), L.MEM_HOST, None))
+    else:
+        bins = np.empty((B, P, 2), dtype=np.int32) if return_bins else None
+        L.check(lib.lkb_bls_power(L.ptr(t), L.ptr(y), L.ptr(dy), L.ptr(offsets), B, L.ptr(period), P, L.ptr(duration),
+                                  D, int(oversample), L.BLS_SNR if objective == "snr" else L.BLS_LIKELIHOOD,
+                                  *[L.ptr(o) for o in outs], L.ptr(bins), L.MEM_HOST, None))
     res = dict(zip(BLS_FIELDS, outs))
     res["period"] = period
     if return_bins:
-        res["bins"] = bins
+        if method == "slow":
+            res["index"] = index
+        else:
+            res["bins"] = bins
     return res
 
 

@@ -537,9 +537,13 @@ class BoxLeastSquaresPeriodogram(Periodogram):
         duration = np.atleast_1d(np.asarray(duration, dtype=np.float64))
         objective = kwargs.pop("objective", None) or "likelihood"
         validate_method(objective, ["likelihood", "snr"])
-        method = kwargs.pop("method", None) or "fast"
-        if method != "fast":
-            raise NotImplementedError("only astropy's method='fast' (binned) BLS is implemented on the GPU")
+        # `bls_method` is the same keyword under a name that to_periodogram("bls", ...) can carry (its first argument
+        # is already called `method`), as `ls_method` is for Lomb-Scargle
+        method, bls_method = kwargs.pop("method", None), kwargs.pop("bls_method", None)
+        method = method or bls_method or "fast"
+        if method not in ("fast", "slow"):
+            raise NotImplementedError("only astropy's methods 'fast' (binned) and 'slow' (exact) are implemented "
+                                      "on the GPU")
         oversample = int(kwargs.pop("oversample", 10))
         if oversample < 1:
             raise ValueError("oversample must be an int greater than 0 (got {})".format(oversample))
@@ -547,8 +551,24 @@ class BoxLeastSquaresPeriodogram(Periodogram):
             raise TypeError("unexpected keyword arguments {}".format(sorted(kwargs)))
         if np.min(period) <= np.max(duration):
             raise ValueError("The maximum transit duration must be shorter than the minimum period")
-        return dict(lc=lc, time=tval, flux=np.asarray(lc.flux.value, dtype=np.float64), dy=dy, period=period,
-                    duration=duration, objective=objective, oversample=oversample, time_unit=time_unit)
+        flux, lc_dy = np.asarray(lc.flux.value, dtype=np.float64), dy
+        if method == "slow" and np.any(np.diff(tval) < 0):
+            # the exact search walks ascending times; its result does not depend on the cadence order (up to the
+            # summation order of the sums)
+            order = np.argsort(tval, kind="stable")
+            tval, flux = tval[order], flux[order]
+            dy = None if dy is None else dy[order]
+        return dict(lc=lc, time=tval, flux=flux, dy=dy, period=period, duration=duration, objective=objective,
+                    oversample=oversample, time_unit=time_unit, method=method, lc_dy=lc_dy)
+
+    @staticmethod
+    def _engine_kwargs(prep):
+        """Keywords of engine.bls_power for a prepared call; `method` only for the exact search, so that the default
+        binned search is requested exactly as by engines that know no other."""
+        kw = dict(oversample=prep["oversample"], objective=prep["objective"])
+        if prep["method"] != "fast":
+            kw["method"] = prep["method"]
+        return kw
 
     @staticmethod
     def _finish(prep, res, b=0):
@@ -564,7 +584,7 @@ class BoxLeastSquaresPeriodogram(Periodogram):
             transit_time=Time(res["transit_time"][b], lc.time.format, lc.time.scale),
             duration=Quantity(res["duration"][b], tu),
             depth=Quantity(res["depth"][b], lc.flux.unit),
-            bls_result={k: res[k][b] for k in res if k not in ("period", "bins")},
+            bls_result={k: res[k][b] for k in res if k not in ("period", "bins", "index")},
             snr=Quantity(res["depth_snr"][b], u.dimensionless_unscaled),
             bls_obj=None,
             time=lc.time,
@@ -576,14 +596,16 @@ class BoxLeastSquaresPeriodogram(Periodogram):
     def from_lightcurve(lc, **kwargs):
         """Creates a Periodogram from a LightCurve using the Box Least Squares method
         (periodogram.py:1042-1192).  Keywords: duration, period, minimum_period, maximum_period,
-        frequency_factor, time_unit, objective, oversample."""
+        frequency_factor, time_unit, objective, oversample, method ("fast": astropy's binned search, K3; "slow": its
+        exact unbinned search, K3s - the reported durations are then the trial durations themselves; through
+        ``to_periodogram("bls", ...)`` spelled ``bls_method``).  Where astropy's method="slow" finds no box with
+        positive depth at a period it raises; here that period gets power -inf."""
         from . import engine
         prep = BoxLeastSquaresPeriodogram._prepare(lc, **kwargs)
         res = engine.bls_power([prep["time"]], [prep["flux"]], None if prep["dy"] is None else [prep["dy"]],
-                               prep["period"], prep["duration"], oversample=prep["oversample"],
-                               objective=prep["objective"])
+                               prep["period"], prep["duration"], **BoxLeastSquaresPeriodogram._engine_kwargs(prep))
         pg = BoxLeastSquaresPeriodogram._finish(prep, res)
-        pg._dy = prep["dy"]
+        pg._dy = prep["lc_dy"]
         return pg
 
     # -- follow-ups ------------------------------------------------------------------------
