@@ -16,15 +16,16 @@
 //   cols   : one CTA = TC columns of one light curve: length-A transforms over n1 in shared memory (in place, one
 //            radix-16 butterfly per thread and pass, twiddles from tables), times exp(2 pi i n2 k1 / Mh), written as
 //            T[lc][c][k1][j] - one contiguous 64 KB block per CTA;
-//   rows   : one CTA = rows k1 = 1 + 8 g .. 8 (g + 1) and their mirror rows A - k1 of one light curve: length-Bc
-//            transforms over n2, then the finish (unpack E / O, deconvolve + tau rotation through one folded table,
+//   rows   : one tile = rows k1 = 1 + 8 g .. 8 (g + 1) and their mirror rows A - k1 of one light curve: length-Bc
+//            transforms over n2 (persistent CTAs, two tiles in flight and the next one arriving: v2_ring), then the finish (unpack E / O, deconvolve + tau rotation through one folded table,
 //            epilogue) -> power, written in 32-byte runs (8 consecutive k1 at one k2 are 8 consecutive frequency
-//            bins); the transform itself never goes back to global memory.  The CTA that would hold row A / 2 twice
+//            bins); the transform itself never goes back to global memory.  The tile that would hold row A / 2 twice
 //            takes row 0 (which mirrors onto itself) instead.
 // All tile geometry is compile-time (template parameter PA): every shared-memory offset inside the passes is
 // `runtime base + constant`.
 #pragma once
 #include "nufft_core.h"
+#include "ptx.cuh"
 
 namespace lkb {
 namespace {
@@ -148,18 +149,39 @@ nufft2_spread_kernel(const int32_t* __restrict__ first_ge, const nufft::Cad* __r
     if (lc0 + q < B) G[(int64_t)(lc0 + q) * cells + e] = make_float2(a0[q], a1[q]);
 }
 
+// ---- who works on a tile -----------------------------------------------------------------------------------------
+// V2Cta: all V2_THREADS threads of a CTA (the double-precision list kernels): __syncthreads, tile loads through
+// registers.  V2Half: group g of the two V2_THREADS-thread groups of a ring CTA (v2_ring): named barrier 1 + g, tile
+// loads as cp.async copies that land while the group computes another tile.
+struct V2Cta {
+  __device__ __forceinline__ int tid() const { return (int)threadIdx.x; }
+  __device__ __forceinline__ void sync() const { __syncthreads(); }
+  template <class CT>
+  __device__ __forceinline__ void put(CT* dst, const CT* src, bool ok) const {
+    *dst = ok ? *src : nufft::CplxOf<CT>::mk(0, 0);
+  }
+};
+struct V2Half {                     // (stateless: the group and the thread index are read afresh, see ptx::tid_x)
+  __device__ __forceinline__ static int group() { return ptx::tid_x() / V2_THREADS; }
+  __device__ __forceinline__ int tid() const { return ptx::tid_x() & (V2_THREADS - 1); }
+  __device__ __forceinline__ void sync() const { ptx::bar_sync_named(1 + group(), V2_THREADS); }
+  __device__ __forceinline__ void put(float2* dst, const float2* src, bool ok) const {
+    ptx::cp_async_8(dst, src, ok ? 8u : 0u);
+  }
+};
+
 // ---- in-place passes over the lines of a tile (compile-time geometry) ---------------------------------------------
 // PLOG: log2 of the line length, LS: skewed line stride, IDX / NS: pass number and the product of earlier radices.
 // nz (first pass only): line positions >= nz hold zeros that were never stored - they are not read either
-template <int PLOG, int LS, int IDX, int NS, class CT = float2>
-__device__ __forceinline__ void v2_pass_t(CT* buf, const CT* __restrict__ tw, int nz = 1 << 30) {
+template <int PLOG, int LS, int IDX, int NS, class CT, class Grp>
+__device__ __forceinline__ void v2_pass_t(CT* buf, const CT* __restrict__ tw, const Grp gp, int nz = 1 << 30) {
   constexpr int R = v2_radix(PLOG, IDX);
   if constexpr (R != 0) {
     constexpr int LR = v2_log2i(R), NB = 16 / R, PNB = PLOG - LR, nb = 1 << PNB;      // nb butterflies per line
     constexpr bool WIDE = nb > V2_THREADS;           // one line, several butterflies of it per thread
     static_assert(WIDE || (V2_THREADS % nb) == 0, "geometry");
     // per-input offset r * nb in the skewed line: v2_in_off<nb>(r)
-    const int t = (int)threadIdx.x;
+    const int t = gp.tid();
     CT u[NB][R];
     int base_in[NB];
 #pragma unroll
@@ -172,7 +194,7 @@ __device__ __forceinline__ void v2_pass_t(CT* buf, const CT* __restrict__ tw, in
       for (int r = 0; r < R; ++r)
         u[q][r] = (IDX > 0 || r * nb < nz) ? buf[base_in[q] + v2_in_off<nb>(r)] : nufft::CplxOf<CT>::mk(0, 0);
     }
-    __syncthreads();
+    gp.sync();
 #pragma unroll
     for (int q = 0; q < NB; ++q) {
       int line, i;
@@ -190,8 +212,8 @@ __device__ __forceinline__ void v2_pass_t(CT* buf, const CT* __restrict__ tw, in
 #pragma unroll
       for (int r = 0; r < R; ++r) buf[base_out + ((NS == 1) ? r : r * (NS + NS / 16))] = u[q][r];
     }
-    __syncthreads();
-    v2_pass_t<PLOG, LS, IDX + 1, NS * R, CT>(buf, tw + ((IDX > 0) ? R * NS : 0));
+    gp.sync();
+    v2_pass_t<PLOG, LS, IDX + 1, NS * R, CT>(buf, tw + ((IDX > 0) ? R * NS : 0), gp);
   }
 }
 
@@ -208,58 +230,76 @@ __device__ __forceinline__ int v2_count(const V2Count nc, int grid_y) {
 }
 
 // ---- cols ---------------------------------------------------------------------------------------------------------
-// grid (Bc / TC, B).  G: pruned fine grids [B][c][n1 < n1max][j]; T: [B][c][k1][j]
-// one transform (light curve slot lc): all threads of the CTA
-template <int PA, class CT>
-__device__ __forceinline__ void v2_cols_one(CT* buf, const CT* __restrict__ G, CT* __restrict__ T, int n1max,
-                                            const CT* __restrict__ tw_a, const CT* __restrict__ t_hi,
-                                            const CT* __restrict__ t_lo, const int64_t lc) {
-  constexpr int A = 1 << PA, PTC = V2_LOG_TILE - PA, TC = 1 << PTC, LS = A + A / 16 + 1, C = V2_BC / TC;
+// G: pruned fine grids [B][c][n1 < n1max][j]; T: [B][c][k1][j].  Tile (lc, c): the TC columns c TC .. of light curve
+// slot lc, one length-A transform per column.
+template <int PA>
+struct V2Cols {
+  static constexpr int A = 1 << PA, PTC = V2_LOG_TILE - PA, TC = 1 << PTC, LS = A + A / 16 + 1, C = V2_BC / TC;
+  static constexpr int ELEMS = TC * LS;                           // points of one tile in shared memory
   // one sweep of the 512 threads covers JW columns x RW rows (RW is a multiple of 16: constant skew increments)
-  constexpr int JW = TC < 32 ? TC : 32, RW = V2_THREADS / JW, CG = TC / JW;
-  constexpr int LJW = JW == 32 ? 5 : JW == 16 ? 4 : JW == 8 ? 3 : JW == 4 ? 2 : JW == 2 ? 1 : 0;
+  static constexpr int JW = TC < 32 ? TC : 32, RW = V2_THREADS / JW, CG = TC / JW;
+  static constexpr int LJW = JW == 32 ? 5 : JW == 16 ? 4 : JW == 8 ? 3 : JW == 4 ? 2 : JW == 2 ? 1 : 0;
   static_assert((1 << LJW) == JW && RW % 16 == 0, "geometry");
-  const int t = (int)threadIdx.x, c = (int)blockIdx.x;
-  const int jl = t & (JW - 1), nl = t >> LJW;
-  const int nvalid = n1max << PTC;
-  const CT* Gp = G + (lc * C + c) * (int64_t)nvalid;
-  const int s_base = jl * LS + v2_skew(nl), g_base = nl * TC + jl;
   // rows the first pass reads: whole input blocks (of A / R1 rows) that contain a row < n1max
-  constexpr int NB1 = A / v2_radix(PA, 0);
-  const int nz = ((n1max + NB1 - 1) / NB1) * NB1;
+  static constexpr int NB1 = A / v2_radix(PA, 0);
+  __device__ __forceinline__ static int nz(int n1max) { return ((n1max + NB1 - 1) / NB1) * NB1; }
+};
+// tile (lc, c) of G -> buf (rows < nz; rows >= n1max as zeros)
+template <int PA, class CT, class Grp>
+__device__ __forceinline__ void v2_cols_load(CT* buf, const CT* __restrict__ G, int n1max, const int64_t lc, const int c,
+                                             const Grp gp) {
+  using Q = V2Cols<PA>;
+  const int t = gp.tid();
+  const int jl = t & (Q::JW - 1), nl = t >> Q::LJW;
+  const int nvalid = n1max << Q::PTC, nz = Q::nz(n1max);
+  const CT* Gp = G + (lc * Q::C + c) * (int64_t)nvalid;
+  const int s_base = jl * Q::LS + v2_skew(nl), g_base = nl * Q::TC + jl;
 #pragma unroll
   for (int u = 0; u < 16; ++u) {
-    const int cg = u % CG, nbk = u / CG;                           // column group, row block of this sweep
-    if (nbk * RW < nz) {
-      const int idx = g_base + nbk * RW * TC + cg * JW;
-      buf[s_base + cg * JW * LS + nbk * (RW + RW / 16)] = (idx < nvalid) ? Gp[idx] : nufft::CplxOf<CT>::mk(0, 0);
+    const int cg = u % Q::CG, nbk = u / Q::CG;                     // column group, row block of this sweep
+    if (nbk * Q::RW < nz) {
+      const int idx = g_base + nbk * Q::RW * Q::TC + cg * Q::JW;
+      gp.put(buf + s_base + cg * Q::JW * Q::LS + nbk * (Q::RW + Q::RW / 16), Gp + (idx < nvalid ? idx : 0), idx < nvalid);
     }
   }
-  __syncthreads();
-  v2_pass_t<PA, LS, 0, 1, CT>(buf, tw_a, nz);
-  CT* Tp = T + (lc * C + c) * (int64_t)V2_TILE;
+}
+// the loaded tile: length-A transforms in shared memory (in place), times exp(2 pi i n2 k1 / Mh) -> T
+template <int PA, class CT, class Grp>
+__device__ __forceinline__ void v2_cols_one(CT* buf, CT* __restrict__ T, int n1max, const CT* __restrict__ tw_a,
+                                            const CT* __restrict__ t_hi, const CT* __restrict__ t_lo, const int64_t lc,
+                                            const int c, const Grp gp) {
+  using Q = V2Cols<PA>;
+  const int t = gp.tid();
+  const int jl = t & (Q::JW - 1), nl = t >> Q::LJW;
+  const int s_base = jl * Q::LS + v2_skew(nl), g_base = nl * Q::TC + jl;
+  v2_pass_t<PA, Q::LS, 0, 1, CT>(buf, tw_a, gp, Q::nz(n1max));
+  CT* Tp = T + (lc * Q::C + c) * (int64_t)V2_TILE;
   const int ph = PA + V2_PB, pl = nufft::v2_log2_lo(ph);
   const unsigned Mmask = (1u << ph) - 1u, lmask = (1u << pl) - 1u;
 #pragma unroll
   for (int u = 0; u < 16; ++u) {
-    const int cg = u % CG, nbk = u / CG;
-    const int k1 = nl + nbk * RW, n2 = c * TC + jl + cg * JW;
+    const int cg = u % Q::CG, nbk = u / Q::CG;
+    const int k1 = nl + nbk * Q::RW, n2 = c * Q::TC + jl + cg * Q::JW;
     const unsigned q = ((unsigned)n2 * (unsigned)k1) & Mmask;       // n2 k1 < 2^22
     const CT wq = nufft::cmul(t_hi[q >> pl], t_lo[q & lmask]);
-    Tp[g_base + nbk * RW * TC + cg * JW] = nufft::cmul(buf[s_base + cg * JW * LS + nbk * (RW + RW / 16)], wq);
+    Tp[g_base + nbk * Q::RW * Q::TC + cg * Q::JW] =
+        nufft::cmul(buf[s_base + cg * Q::JW * Q::LS + nbk * (Q::RW + Q::RW / 16)], wq);
   }
 }
-// grid (Bc / TC, B): one transform per CTA.  (Kept free of any extra kernel parameter: the float2 instantiation sits
-// exactly at the 64-register cap of 2 CTAs/SM, and a 16-byte parameter more made ptxas spill 184 bytes - the column
-// kernel went from 1.12 to 1.66 ms; profiles/launches_r02_c2_escalation_v2_spill.csv.)
-template <int PA, class CT = float2>
-__global__ void __launch_bounds__(V2_THREADS, sizeof(CT) == 8 ? 2 : 1)
-nufft2_cols_kernel(const CT* __restrict__ G, CT* __restrict__ T, int n1max, const CT* __restrict__ tw_a,
-                   const CT* __restrict__ t_hi, const CT* __restrict__ t_lo) {
-  LKB_DYN_SMEM(CT, buf);
-  v2_cols_one<PA, CT>(buf, G, T, n1max, tw_a, t_hi, t_lo, (int64_t)blockIdx.y);
+// grid (Bc / TC, B): one tile per CTA, 2 CTAs/SM.  (Kept free of any extra kernel parameter: it sits exactly at the
+// 64-register cap, and a 16-byte parameter more made ptxas spill 184 bytes - 1.12 -> 1.66 ms,
+// profiles/launches_r02_c2_escalation_v2_spill.csv.  The persistent ring form of v2_ring measured slower here: 1.25
+// instead of 1.13 ms at config 2 on a B200 - the 16 loads a thread has in flight already cover most of the gather.)
+template <int PA>
+__global__ void __launch_bounds__(V2_THREADS, 2)
+nufft2_cols_kernel(const float2* __restrict__ G, float2* __restrict__ T, int n1max, const float2* __restrict__ tw_a,
+                   const float2* __restrict__ t_hi, const float2* __restrict__ t_lo) {
+  LKB_DYN_SMEM(float2, buf);
+  v2_cols_load<PA>(buf, G, n1max, (int64_t)blockIdx.y, (int)blockIdx.x, V2Cta());
+  __syncthreads();
+  v2_cols_one<PA>(buf, T, n1max, tw_a, t_hi, t_lo, (int64_t)blockIdx.y, (int)blockIdx.x, V2Cta());
 }
-// escalation pass (double precision): blocks stride over a device-side count of transforms
+// escalation pass (double precision): grid (Bc / TC, gy); blocks stride over a device-side count of transforms
 template <int PA>
 __global__ void __launch_bounds__(V2_THREADS, 1)
 nufft2_cols_list_kernel(const double2* __restrict__ G, double2* __restrict__ T, int n1max,
@@ -269,10 +309,45 @@ nufft2_cols_list_kernel(const double2* __restrict__ G, double2* __restrict__ T, 
   const int64_t ntr = v2_count(nc, (int)gridDim.y);
   for (int64_t lc = blockIdx.y; lc < ntr; lc += gridDim.y) {
     __syncthreads();
-    v2_cols_one<PA, double2>(buf, G, T, n1max, tw_a, t_hi, t_lo, lc);
+    v2_cols_load<PA>(buf, G, n1max, lc, (int)blockIdx.x, V2Cta());
+    __syncthreads();
+    v2_cols_one<PA>(buf, T, n1max, tw_a, t_hi, t_lo, lc, (int)blockIdx.x, V2Cta());
   }
 }
 
+// ---- persistent ring of tiles (fp32 rows) ----------------------------------------------------------------
+// One CTA of 2 x V2_THREADS threads per SM: two compute groups and three tile buffers in shared memory.  CTA b takes
+// tiles b, b + gridDim.x, ... (local index j = 0, 1, ...); tile j lands in buffer j % 3 and group j % 2 computes it.
+// The group that has finished tile j - past the group barrier after its last read of buffer j % 3 - fetches tile
+// j + 3, the other group's next tile, into that buffer, and goes on to its own tile j + 2, which the other group
+// fetched one step earlier: a tile's global loads overlap the other group's passes.  A fetch is one cp.async per
+// point; its 512 issuing threads arrive (.noinc) on mbarrier j % 6 once their copies have landed, and the computing
+// group waits there.  One mbarrier per (buffer, computing group) and not per buffer: each group then waits on
+// consecutive phases of its own barriers.  (A group sees only every other phase of buffer j % 3, so a parity wait for
+// tile j + 3 made before tile j had landed would pass on the phase before it.)  Epilogue stores stay plain stores.
+// smem: 3 tiles of `elems` points, then the 6 mbarriers.
+template <class Load, class Body>
+__device__ __forceinline__ void v2_ring(float2* smem, const int elems, const int ntiles, Load load, Body body) {
+  uint64_t* bar = reinterpret_cast<uint64_t*>(smem + 3 * elems);
+  const V2Half gp{};
+  if (threadIdx.x < 6) ptx::mbar_init(bar + threadIdx.x, V2_THREADS);
+  __syncthreads();
+  const int b = (int)blockIdx.x, nb = (int)gridDim.x;
+  auto fetch = [&](int j) {
+    if (b + j * nb < ntiles) {
+      load(smem + (j % 3) * elems, b + j * nb, gp);
+      ptx::cp_async_mbar_arrive_noinc(bar + j % 6);
+    }
+  };
+  for (int j = V2Half::group(); j < 3; j += 2) fetch(j);          // group 0: tiles 0 and 2, group 1: tile 1
+  for (int j = V2Half::group(); b + j * nb < ntiles; j += 2) {
+    ptx::mbar_wait(bar + j % 6, (uint32_t)(j / 6) & 1u);
+    body(smem + (j % 3) * elems, b + j * nb, gp);
+    gp.sync();
+    fetch(j + 3);
+  }
+  ptx::cp_async_wait_all();                                        // no copy of this thread outlives it
+}
 // ---- rows + finish -----------------------------------------------------------------------------------------------
 // Folded per-frequency table (built once per call, y-independent): with G d = (C + i S) of a light curve at bin j,
 //   yc + i ys = E d1 + O d2 - ysum c2,   power = yc^2 wz + ys^2 ww
@@ -320,34 +395,43 @@ __device__ __forceinline__ float v2_finish_pw(double2 g1, double2 g2, const V2FT
   return (float)(yc * yc * (double)tb.c.z + ys * ys * (double)tb.c.w);
 }
 
-// MODE 1: finish -> power.  MODE 2: the modes k < nk2_keep * A and their mirrors Mh - k go to Zout [B][Mh] in natural
-// order (the ragged finish kernel reads them there).  One transform (slot lc; lc_base + lc indexes fa.lcmap).
-template <int PA, int MODE, class CT>
-__device__ __forceinline__ void v2_rows_one(CT* buf, const CT* __restrict__ T, const CT* __restrict__ tw_b,
-                                            const V2Finish& fa, CT* __restrict__ Zout, int nk2_keep, const int64_t lc,
-                                            const int lc_base, const int g) {
-  constexpr int A = 1 << PA, PTC = V2_LOG_TILE - PA, TC = 1 << PTC, R = V2_R, LS = V2_LSB, Bc = V2_BC;
-  const int t = (int)threadIdx.x;
-  const bool last = g == (A / (2 * R)) - 1;
-  const int64_t Mh = (int64_t)1 << (PA + V2_PB);
-  auto slot_k1 = [&](int s) -> int {
-    const int h = s >> 3, r = s & (R - 1);
-    if (h == 0) return 1 + g * R + r;
-    if (last && r == 0) return 0;                    // instead of a second copy of row A / 2
-    return A - (g + 1) * R + r;
-  };
-  const CT* Tp = T + lc * Mh;
+// row k1 of slot s (0 .. 15) of row group g: rows 1 + 8 g + r (s = r < 8), then their mirrors A - k1
+template <int PA>
+__device__ __forceinline__ int v2_slot_k1(int s, int g) {
+  constexpr int A = 1 << PA, R = V2_R;
+  const int h = s >> 3, r = s & (R - 1);
+  if (h == 0) return 1 + g * R + r;
+  if (g == (A / (2 * R)) - 1 && r == 0) return 0;    // instead of a second copy of row A / 2
+  return A - (g + 1) * R + r;
+}
+// tile (lc, g) of T -> buf: the 16 rows of row group g of light curve slot lc, one skewed line of Bc points each
+template <int PA, class CT, class Grp>
+__device__ __forceinline__ void v2_rows_load(CT* buf, const CT* __restrict__ T, const int64_t lc, const int g,
+                                             const Grp gp) {
+  constexpr int PTC = V2_LOG_TILE - PA, TC = 1 << PTC, R = V2_R, LS = V2_LSB;
+  const int t = gp.tid();
+  const CT* Tp = T + (lc << (PA + V2_PB));
 #pragma unroll
   for (int u = 0; u < 16; ++u) {
     const int e = t + V2_THREADS * u;
     const int j = e & (TC - 1), r = (e >> PTC) & (R - 1), h = (e >> (PTC + 3)) & 1, c = e >> (PTC + 4);
     const int s = h * R + r;
-    buf[s * LS + v2_skew((c << PTC) + j)] = Tp[(((c << PA) + slot_k1(s)) << PTC) + j];
+    gp.put(buf + s * LS + v2_skew((c << PTC) + j), Tp + ((((c << PA) + v2_slot_k1<PA>(s, g)) << PTC) + j), true);
   }
-  __syncthreads();
-  v2_pass_t<V2_PB, LS, 0, 1, CT>(buf, tw_b);
+}
+// MODE 1: finish -> power.  MODE 2: the modes k < nk2_keep * A and their mirrors Mh - k go to Zout [B][Mh] in natural
+// order (the ragged finish kernel reads them there).  The loaded tile (lc, g) (lc_base + lc indexes fa.lcmap).
+template <int PA, int MODE, class CT, class Grp>
+__device__ __forceinline__ void v2_rows_one(CT* buf, const CT* __restrict__ tw_b, const V2Finish& fa,
+                                            CT* __restrict__ Zout, int nk2_keep, const int64_t lc, const int lc_base,
+                                            const int g, const Grp gp) {
+  constexpr int A = 1 << PA, R = V2_R, LS = V2_LSB, Bc = V2_BC;
+  const int t = gp.tid();
+  const bool last = g == (A / (2 * R)) - 1;
+  const int64_t Mh = (int64_t)1 << (PA + V2_PB);
+  v2_pass_t<V2_PB, LS, 0, 1, CT>(buf, tw_b, gp);
   // one slot per thread for all its items: s = t % 16, k2 = t / 16 + 32 u
-  const int s = t & (2 * R - 1), h = s >> 3, r = s & (R - 1), k1 = slot_k1(s);
+  const int s = t & (2 * R - 1), h = s >> 3, r = s & (R - 1), k1 = v2_slot_k1<PA>(s, g);
   if (MODE == 2) {
     const int keep = nk2_keep < Bc / 2 ? nk2_keep : Bc / 2;
     for (int q = t >> 4; q < 2 * keep; q += V2_THREADS / 16) {
@@ -366,7 +450,9 @@ __device__ __forceinline__ void v2_rows_one(CT* buf, const CT* __restrict__ T, c
   float* prow = fa.power + lcd * fa.F;
   const int64_t jbase = (int64_t)k1 - fa.k0;
   float pmax = 0.0f;
-  constexpr int KSTEP = V2_THREADS / 16, UB = 4;                   // items of a thread: k2 = t / 16 + 32 u
+  // items of a thread: k2 = t / 16 + 32 u, table loads in batches of UB (4 made ptxas spill 124 bytes in the persistent
+  // kernel at its 64-register cap; the ring's other group hides the rest of the latency)
+  constexpr int KSTEP = V2_THREADS / 16, UB = 2;
   for (int k2b = t >> 4; k2b < (int)nK2; k2b += KSTEP * UB) {
     V2FTab tb[UB];
     int64_t jj[UB];
@@ -397,19 +483,8 @@ __device__ __forceinline__ void v2_rows_one(CT* buf, const CT* __restrict__ T, c
   }
 }
 
-// grid (A / 16, B): one transform per CTA (no extra parameters: see nufft2_cols_kernel).  (Tried: the light curve as
-// the FAST block index, so that the CTAs in flight share one 100 KB slice of the finish table - 1.84 ms instead of
-// 1.76 ms: the tile reads of 296 different light curves scatter over DRAM pages, which costs more than the table
-// locality gains.)
-template <int PA, int MODE, class CT = float2>
-__global__ void __launch_bounds__(V2_THREADS, sizeof(CT) == 8 ? 2 : 1)
-nufft2_rows_kernel(const CT* __restrict__ T, const CT* __restrict__ tw_b, V2Finish fa, CT* __restrict__ Zout,
-                   int nk2_keep) {
-  LKB_DYN_SMEM(CT, buf);
-  v2_rows_one<PA, MODE, CT>(buf, T, tw_b, fa, Zout, nk2_keep, (int64_t)blockIdx.y, 0, (int)blockIdx.x);
-}
-// escalation pass (double precision, finish mode): blocks stride over a device-side count of transforms; transform
-// slot lc holds light curve fa.lcmap[nc.base + lc]
+// escalation pass (double precision, finish mode): grid (A / 16, gy); blocks stride over a device-side count of
+// transforms; transform slot lc holds light curve fa.lcmap[nc.base + lc]
 template <int PA>
 __global__ void __launch_bounds__(V2_THREADS, 1)
 nufft2_rows_list_kernel(const double2* __restrict__ T, const double2* __restrict__ tw_b, V2Finish fa, V2Count nc) {
@@ -417,8 +492,26 @@ nufft2_rows_list_kernel(const double2* __restrict__ T, const double2* __restrict
   const int64_t ntr = v2_count(nc, (int)gridDim.y);
   for (int64_t lc = blockIdx.y; lc < ntr; lc += gridDim.y) {
     __syncthreads();
-    v2_rows_one<PA, 1, double2>(buf, T, tw_b, fa, nullptr, 0, lc, nc.base, (int)blockIdx.x);
+    v2_rows_load<PA>(buf, T, lc, (int)blockIdx.x, V2Cta());
+    __syncthreads();
+    v2_rows_one<PA, 1>(buf, tw_b, fa, (double2*)nullptr, 0, lc, nc.base, (int)blockIdx.x, V2Cta());
   }
+}
+// grid (min(SMs, B A / 16)), 1024 threads: tile = lc (A / 16) + g (row group fastest).  (Tried in the one-tile-per-CTA
+// form: the light curve as the fast index, so that the CTAs in flight share one 100 KB slice of the finish table -
+// 1.84 ms instead of 1.76 ms: the tile reads of 296 different light curves scatter over DRAM pages, which costs more
+// than the table locality gains.)
+template <int PA, int MODE>
+__global__ void __launch_bounds__(2 * V2_THREADS, 1)
+nufft2_rows_ring_kernel(const float2* __restrict__ T, const float2* __restrict__ tw_b, V2Finish fa,
+                        float2* __restrict__ Zout, int nk2_keep, int B) {
+  constexpr int NG = (1 << PA) / (2 * V2_R);
+  LKB_DYN_SMEM(float2, smem);
+  v2_ring(smem, 2 * V2_R * V2_LSB, B * NG,
+          [&](float2* buf, int tile, const V2Half gp) { v2_rows_load<PA>(buf, T, tile / NG, tile % NG, gp); },
+          [&](float2* buf, int tile, const V2Half gp) {
+            v2_rows_one<PA, MODE>(buf, tw_b, fa, Zout, nk2_keep, tile / NG, 0, tile % NG, gp);
+          });
 }
 
 // ---- precision escalation -------------------------------------------------------------------------------------
@@ -516,41 +609,51 @@ inline int v2_n1max(int p, int64_t i0_last, int w) {
 }
 inline bool v2_supported(int p) { return p >= V2R_P_MIN && p <= V2R_P_MAX; }
 
+// shared memory of a ring CTA: three tiles of `elems` points and the six mbarriers
+inline size_t v2_ring_smem(int elems) { return 3 * (size_t)elems * sizeof(float2) + 6 * sizeof(uint64_t); }
+// CTAs of a ring launch: one per SM (2 on the CPU emulator), at most one per tile; LKB_NUFFT_RING_CTAS overrides the
+// per-SM count (tests: a forced split of the tiles over CTAs and groups)
+inline unsigned v2_ring_ctas(int64_t ntiles) {
+#if defined(LKB_CUDA_EMU)
+  int64_t n = 2;
+#else
+  int64_t n = sm_count();
+#endif
+  if (const char* e = getenv("LKB_NUFFT_RING_CTAS")) n = std::max(1, atoi(e));
+  return (unsigned)std::max<int64_t>(1, std::min<int64_t>(n, ntiles));
+}
+
 template <int PA, class CT>
 int v2_cols_pa(const CT* G, CT* T, int n1max, int B, const V2TablesT<CT>& tb, cudaStream_t st, V2Count nc) {
-  constexpr int A = 1 << PA, TC = V2_TILE / A;
-  const size_t smem = (size_t)TC * (A + A / 16 + 1) * sizeof(CT);
-  const dim3 grid((unsigned)(V2_BC / TC), (unsigned)B);
-  if constexpr (sizeof(CT) == 16) {
-    if (nc.count) {
-      LKB_CUDA_CHECK(cudaFuncSetAttribute(nufft2_cols_list_kernel<PA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      LKB_LAUNCH_SMEM(grid, V2_THREADS, smem, st, nufft2_cols_list_kernel<PA>)(G, T, n1max, tb.tw_a, tb.t_hi, tb.t_lo, nc);
-      LKB_LAUNCH_CHECK();
-      return LKB_OK;
-    }
+  using Q = V2Cols<PA>;
+  const size_t smem = (size_t)Q::ELEMS * sizeof(CT);
+  const dim3 grid((unsigned)Q::C, (unsigned)B);
+  if constexpr (sizeof(CT) == 16) {                  // the escalation pass
+    LKB_CUDA_CHECK(cudaFuncSetAttribute(nufft2_cols_list_kernel<PA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    LKB_LAUNCH_SMEM(grid, V2_THREADS, smem, st, nufft2_cols_list_kernel<PA>)(G, T, n1max, tb.tw_a, tb.t_hi, tb.t_lo, nc);
+  } else {
+    LKB_CUDA_CHECK(cudaFuncSetAttribute(nufft2_cols_kernel<PA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    LKB_LAUNCH_SMEM(grid, V2_THREADS, smem, st, nufft2_cols_kernel<PA>)(G, T, n1max, tb.tw_a, tb.t_hi, tb.t_lo);
   }
-  LKB_CUDA_CHECK(cudaFuncSetAttribute(nufft2_cols_kernel<PA, CT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  LKB_LAUNCH_SMEM(grid, V2_THREADS, smem, st, nufft2_cols_kernel<PA, CT>)(G, T, n1max, tb.tw_a, tb.t_hi, tb.t_lo);
   LKB_LAUNCH_CHECK();
   return LKB_OK;
 }
 template <int PA, class CT>
 int v2_rows_pa(const CT* T, int B, const V2TablesT<CT>& tb, const V2Finish* fa, CT* Zout, int nk2_keep, cudaStream_t st,
                V2Count nc) {
-  const size_t smem = (size_t)(2 * V2_R) * V2_LSB * sizeof(CT);
-  const dim3 grid((unsigned)((1 << PA) / (2 * V2_R)), (unsigned)B);
-  if constexpr (sizeof(CT) == 16) {
-    if (nc.count && fa) {
-      LKB_CUDA_CHECK(cudaFuncSetAttribute(nufft2_rows_list_kernel<PA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      LKB_LAUNCH_SMEM(grid, V2_THREADS, smem, st, nufft2_rows_list_kernel<PA>)(T, tb.tw_b, *fa, nc);
-      LKB_LAUNCH_CHECK();
-      return LKB_OK;
-    }
+  constexpr int NG = (1 << PA) / (2 * V2_R);
+  if constexpr (sizeof(CT) == 16) {                  // the escalation pass: always the finish
+    const size_t smem = (size_t)(2 * V2_R) * V2_LSB * sizeof(CT);
+    LKB_CUDA_CHECK(cudaFuncSetAttribute(nufft2_rows_list_kernel<PA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    LKB_LAUNCH_SMEM(dim3((unsigned)NG, (unsigned)B), V2_THREADS, smem, st, nufft2_rows_list_kernel<PA>)(T, tb.tw_b, *fa, nc);
+  } else {
+    const size_t smem = v2_ring_smem(2 * V2_R * V2_LSB);
+    const unsigned grid = v2_ring_ctas((int64_t)B * NG);
+    LKB_CUDA_CHECK(cudaFuncSetAttribute(nufft2_rows_ring_kernel<PA, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    LKB_CUDA_CHECK(cudaFuncSetAttribute(nufft2_rows_ring_kernel<PA, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (fa) LKB_LAUNCH_SMEM(grid, 2 * V2_THREADS, smem, st, nufft2_rows_ring_kernel<PA, 1>)(T, tb.tw_b, *fa, nullptr, 0, B);
+    else LKB_LAUNCH_SMEM(grid, 2 * V2_THREADS, smem, st, nufft2_rows_ring_kernel<PA, 2>)(T, tb.tw_b, V2Finish(), Zout, nk2_keep, B);
   }
-  LKB_CUDA_CHECK(cudaFuncSetAttribute(nufft2_rows_kernel<PA, 1, CT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  LKB_CUDA_CHECK(cudaFuncSetAttribute(nufft2_rows_kernel<PA, 2, CT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  if (fa) LKB_LAUNCH_SMEM(grid, V2_THREADS, smem, st, nufft2_rows_kernel<PA, 1, CT>)(T, tb.tw_b, *fa, nullptr, 0);
-  else LKB_LAUNCH_SMEM(grid, V2_THREADS, smem, st, nufft2_rows_kernel<PA, 2, CT>)(T, tb.tw_b, V2Finish(), Zout, nk2_keep);
   LKB_LAUNCH_CHECK();
   return LKB_OK;
 }

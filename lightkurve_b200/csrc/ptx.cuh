@@ -1,5 +1,8 @@
-// Inline-PTX wrappers for sm_100a: mbarrier, TMA bulk copies, tcgen05 / TMEM.
+// Inline-PTX wrappers for sm_100a: mbarrier, named barriers, cp.async, TMA bulk copies, tcgen05 / TMEM.
+// Under the CPU emulator (LKB_CUDA_EMU, tests/native/cuda_emu.h) the few that ls_nufft.cu uses have host versions at
+// the end of this file.
 #pragma once
+#if !defined(LKB_CUDA_EMU)
 #include <stdint.h>
 #include <cuda.h>
 
@@ -63,6 +66,34 @@ __device__ __forceinline__ void mbar_wait_sleep(uint64_t* bar, uint32_t parity, 
     if (ns) __nanosleep(ns);
   }
 }
+
+// %tid.x read afresh at each call (volatile: not hoisted out of a loop).  In a persistent kernel the compiler would
+// otherwise keep every per-thread offset derived from it live across the whole loop body - at a register cap, in local
+// memory.
+__device__ __forceinline__ int tid_x() {
+  int t;
+  asm volatile("mov.u32 %0, %%tid.x;" : "=r"(t));
+  return t;
+}
+
+// ---- named barriers / cp.async ---------------------------------------------------
+// barrier `id` (1 .. 15) over `nthreads` threads (a multiple of 32) of the CTA
+__device__ __forceinline__ void bar_sync_named(int id, int nthreads) {
+  asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
+}
+// 8-byte copy global -> shared (SASS: LDGSTS); src_bytes = 0 zero-fills the destination and reads nothing
+__device__ __forceinline__ void cp_async_8(void* dst_smem, const void* src_gmem, uint32_t src_bytes) {
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 8, %2;" ::"r"(smem_u32(dst_smem)), "l"(src_gmem), "r"(src_bytes)
+               : "memory");
+}
+// one arrival on `bar` once every cp.async this thread has issued so far has landed; the arrival is one of the count
+// the barrier was initialised with (.noinc)
+__device__ __forceinline__ void cp_async_mbar_arrive_noinc(uint64_t* bar) {
+  asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
+}
+
+// wait until every cp.async this thread has issued has landed
+__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
 // ---- async-proxy fences / TMA ---------------------------------------------------
 __device__ __forceinline__ void fence_proxy_async_smem() {
@@ -223,3 +254,71 @@ __device__ __forceinline__ void umma_commit_2cta(uint64_t* bar) {
 
 }  // namespace ptx
 }  // namespace lkb
+
+#else  // LKB_CUDA_EMU
+// Host versions for the CPU emulator, which runs every thread of a block as a host thread and one block at a time, so
+// state shared by all blocks is the state of the running block.  The kernels run the same ring logic - buffer indices,
+// parities, group handoff - as on the device.
+// mbarrier word: bits 0-31 the arrival count it was initialised with, 32-62 arrivals still pending in the current
+// phase, 63 the current phase's parity.  A parity wait returns once the phase of that parity has completed, i.e. while
+// the current phase's parity differs - so, as on the device, a wait two phases ahead passes on the phase before.
+// cp.async is a synchronous copy, so the arrive that tracks it is a plain arrive.
+#include <stdint.h>
+#include <string.h>
+#include <condition_variable>
+#include <mutex>
+
+namespace lkb {
+namespace ptx {
+struct EmuSync {
+  std::mutex m;
+  std::condition_variable cv;
+  int arrived[16] = {};
+  long generation[16] = {};
+};
+inline EmuSync& emu_sync() {
+  static EmuSync s;
+  return s;
+}
+inline int tid_x() { return (int)threadIdx.x; }
+inline void bar_sync_named(int id, int nthreads) {
+  EmuSync& e = emu_sync();
+  std::unique_lock<std::mutex> lk(e.m);
+  const long gen = e.generation[id];
+  if (++e.arrived[id] == nthreads) {
+    e.arrived[id] = 0;
+    ++e.generation[id];
+    e.cv.notify_all();
+    return;
+  }
+  e.cv.wait(lk, [&] { return gen != e.generation[id]; });
+}
+inline void mbar_init(uint64_t* bar, uint32_t count) {
+  std::lock_guard<std::mutex> lk(emu_sync().m);
+  *bar = (uint64_t)count | ((uint64_t)count << 32);
+}
+inline void mbar_arrive(uint64_t* bar) {
+  EmuSync& e = emu_sync();
+  std::lock_guard<std::mutex> lk(e.m);
+  const uint64_t count = *bar & 0xffffffffull, phase = *bar >> 63, pending = ((*bar >> 32) & 0x7fffffffull) - 1;
+  if (pending == 0) {
+    *bar = count | (count << 32) | ((phase ^ 1ull) << 63);
+    e.cv.notify_all();
+  } else {
+    *bar = count | (pending << 32) | (phase << 63);
+  }
+}
+inline void mbar_wait(uint64_t* bar, uint32_t parity) {
+  EmuSync& e = emu_sync();
+  std::unique_lock<std::mutex> lk(e.m);
+  e.cv.wait(lk, [&] { return (uint32_t)(*bar >> 63) != (parity & 1u); });
+}
+inline void cp_async_8(void* dst_smem, const void* src_gmem, uint32_t src_bytes) {
+  memset(dst_smem, 0, 8);
+  if (src_bytes) memcpy(dst_smem, src_gmem, src_bytes);
+}
+inline void cp_async_mbar_arrive_noinc(uint64_t* bar) { mbar_arrive(bar); }
+inline void cp_async_wait_all() {}
+}  // namespace ptx
+}  // namespace lkb
+#endif  // LKB_CUDA_EMU
